@@ -6,7 +6,8 @@ A "step" is one pass of the hot path over one synthetic assay: WT of L=512 resid
 (SURVEY.md §8d config 2): 512 masked copies x 514 tokens through 33 layers, masked-row LM head, mutant scoring.
 
   python bench.py --gpus N --steps K --warmup W            # our arm  (one JSON line on rank 0)
-  python bench.py --impl reference --gpus N ...            # reference arm: the reference's CPU path on the host cores
+  python bench.py ... --dump-outputs DIR                   # + DIR/scores.npy: the scores of the last timed step, to compare builds
+  python bench.py --impl reference --gpus N ...            # reference arm: the reference's CPU loop (oracle port) on the host cores
 
 `value`  : whole-job mutants/s with inputs already resident in HBM (device-timed with CUDA events, max over ranks; no profiling
            events inside this leg).
@@ -56,6 +57,9 @@ def parse():
     ap.add_argument("--no-other-modes", action="store_true", help="skip the legs at the other precision modes")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
     ap.add_argument("--small", action="store_true", help="tiny model/assay (debugging only; not a valid bench)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the per-mutant scores of the last timed step (rank 0, headline precision) to DIR/scores.npy (float32); "
+                         "inputs are seeded, so runs with the same arguments score the same assay")
     return ap.parse_args()
 
 
@@ -158,35 +162,15 @@ _CPU_CACHE = {}
 
 
 def _cpu_forward_fn(arch, state):
-    """-> (kind, fn(tokens[1,T]) -> logits): the UNMODIFIED reference model when the reference tree is present
-    (PG_REFERENCE_ROOT or /root/reference; oracle/ref_shims.py), else the oracle port of it."""
+    """-> (kind, fn(tokens[1,T]) -> logits): the oracle port of the reference forward (oracle/esm_oracle.py), so the CPU arm
+    runs from this repository alone."""
     if "fwd" in _CPU_CACHE:
         return _CPU_CACHE["fwd"]
     from oracle import esm_oracle as O
-    from oracle import ref_shims
-    from proteingym_b200 import synth
     kind = "esm2" if arch.kind == "esm2" else "esm1v"
-    fn = None
-    which = "port"
-    if ref_shims.available() and not os.environ.get("PG_BENCH_CPU_PORT"):
-        try:
-            import shutil
-            import tempfile
-            mod = ref_shims.install()
-            tmp = tempfile.mkdtemp(prefix="pg_bench_ref_")
-            path = os.path.join(tmp, "esm2_bench.pt" if kind == "esm2" else "esm1v_bench.pt")
-            synth.write_esm_checkpoint(path, arch, state={k: v for k, v in state.items()})
-            model, _ = mod.pretrained.load_model_and_alphabet(path)
-            model.eval()
-            shutil.rmtree(tmp, ignore_errors=True)
-            fn = lambda toks: model(toks)["logits"]
-            which = "reference"
-        except Exception as e:  # noqa: BLE001
-            log(f"reference model unavailable ({type(e).__name__}: {e}); timing the oracle port")
-    if fn is None:
-        st = O.load_state(state, kind, torch.float32)
-        fn = lambda toks: O.esm_forward(st, toks, kind, arch.layers, arch.heads, arch.token_dropout)
-    _CPU_CACHE["fwd"] = (which, fn)
+    st = O.load_state(state, kind, torch.float32)
+    fn = lambda toks: O.esm_forward(st, toks, kind, arch.layers, arch.heads, arch.token_dropout)
+    _CPU_CACHE["fwd"] = ("port", fn)
     return _CPU_CACHE["fwd"]
 
 
@@ -229,7 +213,7 @@ def cpu_mutants_per_s(arch, state, seconds, threads, L, n_mut):
 
 def cpu_sample_text(info):
     return (f"{info['forwards_timed']} batch-1 masked forwards of T={info['T']} (median {info['t_forward_s']:.3f} s each, "
-            f"{'unmodified reference ProteinBertModel/ESM2' if info['kind'] == 'reference' else 'oracle port of the reference forward'}) "
+            "oracle port of the reference forward) "
             f"extrapolated x{info['T']} = the reference's L+2 forwards per assay")
 
 
@@ -521,7 +505,8 @@ def main():
         clocks = sampler.window(t_host0, t_host1) if sampler else None
         res = {"value": world * a.steps * n_mut / (ms_total / 1e3), "ms_per_step": ms_total / a.steps, "gpu_launches": int(launches),
                "clocks": clocks, "weight_load_s": load_s,
-               "per_rank_ms": {"min": min(per_rank), "median": statistics.median(per_rank), "max": max(per_rank)}}
+               "per_rank_ms": {"min": min(per_rank), "median": statistics.median(per_rank), "max": max(per_rank)},
+               "last_scores": outs[-1].cpu().numpy()}
         # ---- leg 2: the same K steps with a CUDA-event pair around every kernel -> per-kernel times for the roofline ----
         log(f"measure {precision}: roofline leg")
         barrier()
@@ -618,6 +603,9 @@ def main():
 
     cpu_state = {k: v.cpu() for k, v in state.items()} if (rank == 0 and world == 1 and not a.no_cpu_baseline) else None
     main_res = measure(a.precision, with_e2e=True)
+    if a.dump_outputs and rank == 0:
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        np.save(os.path.join(a.dump_outputs, "scores.npy"), main_res["last_scores"].astype(np.float32))
     others = [] if (a.small or a.no_other_modes) else [(m, measure(m, with_e2e=False)) for m in ("f16d", "f16f8", "f16x3", "f16") if m != a.precision]
     del state
     torch.cuda.empty_cache()
